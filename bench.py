@@ -58,7 +58,15 @@ def parse_args():
     ap.add_argument("--merge", choices=["allreduce", "gather"], default="allreduce",
                     help="N>1 merge of the partial aggregates: in-place all-reduce of the dense slot arrays (SURVEY 8e) or "
                          "gather of partial rows to rank 0 + final aggregate (the reference plan's UNPARTITIONED exchange)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="q41 GPU arm: after the timed steps, write the result columns of the last timed step as DIR/<name>.npy "
+                         "(float64, rows sorted by group key) so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.workload != "q41" or args.impl != "gpu"):
+        ap.error("--dump-outputs is implemented for the q41 workload of the GPU arm")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -291,6 +299,19 @@ def run_reference(args):
 # ---------------------------------------------------------------------------------------------------
 # GPU arm
 # ---------------------------------------------------------------------------------------------------
+def dump_outputs(out_dir, result, names):
+    """result columns (chunk_out_to_host form) -> out_dir/<names[slot]>.npy, float64 with NULL as NaN.  The rows are sorted
+    by all columns, group keys first: the order in which the aggregate emits its groups is not part of the result."""
+    from starrocks_b200.rows import gpu_rows
+    rows = gpu_rows(result)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, (slot, _, _, _) in enumerate(result):
+        vals = [r[k] for r in rows]
+        if any(v is not None and float(v) != v for v in vals):
+            raise SystemExit(f"bench.py: column {names[slot]} is not exact in float64; refusing to dump a rounded value")
+        np.save(os.path.join(out_dir, names[slot] + ".npy"), np.array([np.nan if v is None else v for v in vals], dtype=np.float64))
+
+
 def run_gpu(args):
     import torch
     import torch.distributed as dist
@@ -415,6 +436,9 @@ def run_gpu(args):
     ms_per_step = elapsed_ms / args.steps
     value = n * world / (ms_per_step / 1000.0)
     rows_passed = frag.rows_passed
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, result, {ssb.D_YEAR: "d_year", ssb.C_NATION: "c_nation",
+                                                 ssb.OUT_SUM_REVENUE: "sum_lo_revenue", ssb.OUT_SUM_SUPPLYCOST: "sum_lo_supplycost"})
 
     # ---- e2e: host (pinned) column buffers through the same C-ABI call, H2D inside the timed region ----
     e2e = None

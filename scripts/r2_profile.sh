@@ -1,26 +1,12 @@
 #!/bin/bash
-# round-2 profiling pass on the GPU box (one gpurun call): TMA experiment, launch list, ncu --set full of the hot kernels.
+# round-2 profiling pass on a B200 in one run: launch list, ncu --set full of the hot kernels.
 # outputs under gpurun_out/ (summaries are copied to profiles/ afterwards)
 set -x
 cd "$(dirname "$0")/.."
 mkdir -p gpurun_out
-# 1. TMA-staged stream pass: correctness + timing against the LDG form
-SR_FRAG_STREAM_TMA=1 timeout 300 python -m pytest tests/test_gpu_parity.py -x -q -m gpu -k "frag" 2>&1 | tail -3
-timeout 300 python bench.py --steps 20 --warmup 5 --no-e2e --no-cpu-baseline > gpurun_out/r2_bench_ldg.json 2>/dev/null
-SR_FRAG_STREAM_TMA=1 timeout 300 python bench.py --steps 20 --warmup 5 --no-e2e --no-cpu-baseline > gpurun_out/r2_bench_tma.json 2>/dev/null
-python - <<'PY'
-import json
-for nm in ("ldg", "tma"):
-    try:
-        d = json.loads(open(f"gpurun_out/r2_bench_{nm}.json").read().strip().splitlines()[-1])
-        print(nm, "ms_per_step", d["ms_per_step"], [(k["name"], round(k["ms"], 4)) for k in d["roofline"]["kernels"]], "read_peak", d["roofline"].get("peak_read_only"))
-    except Exception as e:
-        print(nm, "failed", e)
-PY
-# 2. launch list of the default bench command
+# 1. launch list of the default bench command
 timeout 600 ncu --metrics gpu__time_duration.sum --clock-control none -c 600 --csv --log-file gpurun_out/r2_launches.csv python bench.py --steps 2 --warmup 1 --no-e2e --no-cpu-baseline > gpurun_out/r2_launches_bench.log 2>&1
-# 3. full capture of the fragment kernels (LDG form and TMA form) and of the partitioned aggregate
+# 2. full capture of the fragment kernels and of the partitioned aggregate
 timeout 600 ncu --set full --clock-control none --import-source on -k regex:k_frag_ -c 3 -o gpurun_out/r2_frag python bench.py --steps 1 --warmup 1 --no-e2e --no-cpu-baseline > gpurun_out/r2_frag_ncu.log 2>&1
-SR_FRAG_STREAM_TMA=1 timeout 600 ncu --set full --clock-control none --import-source on -k regex:k_frag_stream -c 1 -o gpurun_out/r2_frag_tma python bench.py --steps 1 --warmup 1 --no-e2e --no-cpu-baseline > gpurun_out/r2_frag_tma_ncu.log 2>&1
 timeout 600 ncu --set full --clock-control none --import-source on -k regex:k_aggp -c 4 -o gpurun_out/r2_aggp python tools/groupby_highcard.py --rows 200000000 --keys 20000000 --reps 1 > gpurun_out/r2_aggp_ncu.log 2>&1
 ls -la gpurun_out | tail -12

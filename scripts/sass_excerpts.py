@@ -49,8 +49,6 @@ print("SASS excerpts of the hot kernels (cuobjdump -sass starrocks_b200/libsr_gp
 section("k_frag_stream_tests<false> (streaming pass, LDG form): 128-bit streaming loads of the two key columns (LDG.E.NA.128), bitmap word fetches from "
         "shared memory (LDS) and global memory (predicated LDG.E.CONSTANT), clamp onto the guard bit (VIMNMX / VIADDMNMX), selection-vector stores",
         "k_frag_stream_testsILb0", [r"LDG\.E\.NA\.128", r"@P\d\s+LDG\.E\.CONSTANT", r"VIMNMX|VIADDMNMX", r"STG\.E\.64", r"VOTE|POPC"])
-section("k_frag_stream_tests_tma<false> (TMA-staged variant, opt-in SR_FRAG_STREAM_TMA): bulk copies into shared memory (UBLKCP), mbarrier phases (SYNCS)",
-        "k_frag_stream_tests_tma", [r"UBLKCP", r"SYNCS", r"LDS\.128", r"FENCE"])
 section("k_frag_gather_join (selection-vector pass of one join): sector gathers of the key column through the selection vector", "k_frag_gather_join",
         [r"LDG", r"STG", r"VOTE|POPC", r"ATOMG"], 16)
 section("k_frag_gather_agg<SMEM_AGG=true> (final pass): dependent gathers, shared-memory accumulators (ATOMS / REDS on 32-bit halves)", "k_frag_gather_aggILb1ELb0",

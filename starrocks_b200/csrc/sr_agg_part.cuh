@@ -75,8 +75,6 @@ struct ScatterArgs {
     unsigned long long ovf_cap;
     int32_t fan_bits;                    // log2 of this level's fan-out
     int32_t local_shift;                 // local bucket = (bucket >> local_shift) & (fan - 1)
-    int32_t l2_prefetch;                 // level 1 from plain columns: request the CTA's NEXT tile into L2 meanwhile
-    int32_t pad;
 };
 
 // ask L2 for the 128-byte lines of [p, p + bytes): one line per thread and step (sequential input only -- a prefetch
@@ -206,9 +204,9 @@ __global__ void __launch_bounds__(AGGP_BLOCK, 1024 / AGGP_BLOCK) k_aggp_scatter(
         int tile_n;
         uint32_t cbase;
         locate(tile, row0, tile_n, cbase);
-        if (sa.l2_prefetch && MODE == SCATTER_CHUNK_SIMPLE && tile + gridDim.x < ntiles) {
+        if (MODE == SCATTER_CHUNK_SIMPLE && tile + gridDim.x < ntiles) {
             // the input columns of the CTA's NEXT tile are requested into L2 while this tile is ranked, scanned and copied
-            // out.  Measured per 1e9 rows (SR_AGG_NO_L2_PREFETCH=1 switches it off): level 1 11.90 -> 11.47 ms.  The same
+            // out.  Measured per 1e9 rows against the same kernel without it: level 1 11.90 -> 11.47 ms.  The same
             // prefetch on the record tiles of level 2 and on the next bucket of the apply pass cost 0.5 ms each (8.09 ->
             // 8.65, 9.94 -> 10.40 ms: their input was written by the previous kernel and is largely L2-resident already,
             // the prefetch instructions only compete for issue slots) and is not done.

@@ -166,7 +166,6 @@ static int32_t agg_push_partitioned(sr_agg* a, const VTab& vt, int64_t n, bool f
             pl.bucket_shift = log2cap - log2p;
         }
         pl.bits2 = pl.bits > srd::AGGP_MAX_FAN_BITS ? pl.bits / 2 : 0;
-        if (pl.bits2 && getenv("SR_AGG_BITS2")) pl.bits2 = std::min(std::max(atoi(getenv("SR_AGG_BITS2")), pl.bits - srd::AGGP_MAX_FAN_BITS), srd::AGGP_MAX_FAN_BITS); // tuning knob
         const int P = 1 << pl.bits;
         const int F1 = 1 << (pl.bits - pl.bits2);
         pl.cap2 = aggp_region_cap((double)m / P);
@@ -196,9 +195,6 @@ static int32_t agg_push_partitioned(sr_agg* a, const VTab& vt, int64_t n, bool f
         sa.ovf = a->part_ovf.as<unsigned long long>();
         sa.ovf_count = ovf_count;
         sa.ovf_cap = (unsigned long long)m;
-        static const bool no_prefetch = getenv("SR_AGG_NO_L2_PREFETCH") != nullptr; // A/B switch of the next-tile L2 prefetch
-        sa.l2_prefetch = no_prefetch ? 0 : 1;
-        sa.pad = 0;
         if (pl.bits2 == 0) {
             sa.cursor = cursor;
             sa.dst = rec_final;

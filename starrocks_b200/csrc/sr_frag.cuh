@@ -328,29 +328,6 @@ static int32_t frag_plan(sr_fragment* f, const VTab& vt, int64_t n) {
             if (ok && nt > 1) reach1 = f->pass.tests[0].kind == 0 ? (double)counts[16] / (double)std::max<int64_t>(sample, 1) : f->pred_rate * f->pass_rate[ord[0]];
             f->pass.num_vec = (ok && nt > 1 && reach1 >= 0.08) ? 2 : 1;
         }
-        // fact values the final pass reads: keys of the joins it looks up or tests, group keys, aggregate inputs
-        {
-            std::vector<int> need;
-            auto want = [&](int id) {
-                if (id >= 0 && id < (int)f->value_src.size() && f->value_src[id] < 0 && std::find(need.begin(), need.end(), id) == need.end()) need.push_back(id);
-            };
-            for (int q = 0; q < f->num_joins; q++)
-                if (h.joins[q].need_head || q >= ff) want(h.joins[q].key_value_id);
-            const srd::AggDev& ah = f->agg->host;
-            for (int k = 0; k < ah.num_keys; k++) want(ah.key_value_id[k]);
-            for (int q = 0; q < ah.num_fns; q++)
-                for (int k = 0; k < ah.fns[q].input.num_nodes; k++)
-                    if (ah.fns[q].input.nodes[k].op == srd::C_LOAD_I || ah.fns[q].input.nodes[k].op == srd::C_LOAD_D) want(ah.fns[q].input.nodes[k].arg);
-            for (int k = 0; k < SR_FINAL_PREFETCH; k++) f->pass.final_vals[k] = -1;
-            for (int k = 0; k < SR_MAX_VALUES; k++) f->pass.final_slot[k] = -1;
-            // measured on B200 (profiles/r1_notes.md): the burst costs more issue slots and registers than the
-            // latency it hides -- the final pass is L1TEX-gather bound, not latency bound -- so it stays off
-            const bool kFinalPrefetch = false;
-            for (size_t k = 0; k < need.size() && k < SR_FINAL_PREFETCH; k++) {
-                f->pass.final_vals[k] = (int8_t)need[k]; // also the L2 prefetch list of host-resident input
-                if (kFinalPrefetch) f->pass.final_slot[need[k]] = (int8_t)k;
-            }
-        }
         f->gather_joins.clear();
         for (int q = ns; q < ff; q++) f->gather_joins.push_back(q);
         // streaming pass shared memory: bitmaps of the streamed joins only
@@ -471,8 +448,8 @@ static int32_t frag_push(sr_fragment* f, const sr_chunk_view* fact) {
         if (!f->gather_joins.empty()) SR_TRY(f->sel[1].reserve(ctx, sizeof(srd::SelEntry) * ((size_t)n + slack)));
         // this push's pass parameters: the carried key (planned in f->pass) is only used for host-resident input
         srd::PassDev pass = f->pass;
-        pass.host_input = fact->mem == SR_MEM_HOST_PINNED ? 1 : 0;
-        const bool carry = pass.host_input && pass.carry_join >= 0; // (HBM input, measured: stream +0.27 ms, final -0.09 ms)
+        const bool pinned_input = fact->mem == SR_MEM_HOST_PINNED;
+        const bool carry = pinned_input && pass.carry_join >= 0; // (HBM input, measured: stream +0.27 ms, final -0.09 ms)
         if (!carry) pass.carry_join = pass.carry_value_id = -1;
         unsigned long long* cnt = f->pass_counters.as<unsigned long long>();
         SR_CUDA(ctx, cudaMemsetAsync(cnt, 0, 16 * sizeof(uint64_t), ctx->stream));
@@ -488,16 +465,7 @@ static int32_t frag_push(sr_fragment* f, const sr_chunk_view* fact) {
             const VDesc& d = vt.v[pass.tests[t].value_id];
             if (d.nulls != nullptr || (t < pass.num_vec && (((uintptr_t)d.data) & 15) != 0)) tests = false;
         }
-        static const bool use_tma = getenv("SR_FRAG_STREAM_TMA") != nullptr; // experiment: TMA-staged vector columns
-        if (tests && use_tma && !pass.host_input) {
-            const uint32_t bitmap_bytes = (uint32_t)((f->stream_smem + 127) / 128 * 128);
-            const size_t sm = bitmap_bytes + srd::STREAM_TMA_SMEM;
-            SR_CUDA(ctx, cudaFuncSetAttribute(srd::k_frag_stream_tests_tma<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-            int per_sm = 1;
-            SR_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, srd::k_frag_stream_tests_tma<false>, srd::STREAM_BLOCK, sm));
-            const int tgrid = (int)std::min<int64_t>((int64_t)std::max(per_sm, 1) * ctx->num_sms, (n + srd::STREAM_TILE - 1) / srd::STREAM_TILE);
-            srd::k_frag_stream_tests_tma<false><<<tgrid, srd::STREAM_BLOCK, sm, ctx->stream>>>(fdev, pass, vt, n, bitmap_bytes, f->sel[0].as<srd::SelEntry>(), cnt);
-        } else if (tests) {
+        if (tests) {
             if (carry)
                 srd::k_frag_stream_tests<true><<<sgrid, srd::STREAM_BLOCK, f->stream_smem, ctx->stream>>>(fdev, pass, vt, n, f->sel[0].as<srd::SelEntry>(), cnt);
             else
@@ -518,23 +486,26 @@ static int32_t frag_push(sr_fragment* f, const sr_chunk_view* fact) {
             k++;
         }
         SR_CUDA(ctx, cudaEventRecord(f->ev[2], ctx->stream));
+        // the final pass over sel_in[0, *n_in); rows the hash table refuses are appended to fail_list (nullptr: no hash
+        // table).  Only a dense table is accumulated in shared memory (agg_compile), so a hash table always takes
+        // k_frag_gather_agg<false> or the expand kernel, the first pass and its retries alike.
+        auto final_pass = [&](const srd::SelEntry* sel_in, const unsigned long long* n_in, srd::SelEntry* fail_list,
+                              unsigned long long* fail_count) -> int32_t {
+            const srd::AggDev* adev = (const srd::AggDev*)a->dev.p;
+            if (f->expand)
+                srd::k_frag_gather_agg_expand<<<f->final_grid, srd::GATHER_BLOCK, 0, ctx->stream>>>(fdev, adev, pass, vt, sel_in, n_in, fail_list, fail_count);
+            else if (ah.num_keys == 0)
+                srd::k_frag_gather_agg<false, true><<<f->final_grid, srd::GATHER_BLOCK, 0, ctx->stream>>>(fdev, adev, pass, vt, sel_in, n_in, fail_list, fail_count);
+            else if (f->smem_agg)
+                srd::k_frag_gather_agg<true><<<f->final_grid, srd::GATHER_BLOCK, a->smem_bytes, ctx->stream>>>(fdev, adev, pass, vt, sel_in, n_in, fail_list, fail_count);
+            else
+                srd::k_frag_gather_agg<false><<<f->final_grid, srd::GATHER_BLOCK, 0, ctx->stream>>>(fdev, adev, pass, vt, sel_in, n_in, fail_list, fail_count);
+            SR_LAUNCH_CHECK(ctx);
+            return SR_OK;
+        };
         // hash table: rows it refuses go to the other selection buffer (free by now) and are retried after a growth
         if (hash) SR_TRY(f->sel[cur ^ 1].reserve(ctx, sizeof(srd::SelEntry) * ((size_t)n + slack)));
-        srd::SelEntry* fail_list = hash ? f->sel[cur ^ 1].as<srd::SelEntry>() : nullptr;
-        unsigned long long* fail_count = cnt + 8;
-        if (f->expand)
-            srd::k_frag_gather_agg_expand<<<f->final_grid, srd::GATHER_BLOCK, 0, ctx->stream>>>(fdev, (const srd::AggDev*)a->dev.p, pass, vt,
-                                                                                       f->sel[cur].as<srd::SelEntry>(), cnt + k, fail_list, fail_count);
-        else if (ah.num_keys == 0)
-            srd::k_frag_gather_agg<false, true><<<f->final_grid, srd::GATHER_BLOCK, 0, ctx->stream>>>(fdev, (const srd::AggDev*)a->dev.p, pass, vt,
-                                                                                              f->sel[cur].as<srd::SelEntry>(), cnt + k, nullptr, nullptr);
-        else if (f->smem_agg)
-            srd::k_frag_gather_agg<true><<<f->final_grid, srd::GATHER_BLOCK, a->smem_bytes, ctx->stream>>>(fdev, (const srd::AggDev*)a->dev.p, pass, vt,
-                                                                                                   f->sel[cur].as<srd::SelEntry>(), cnt + k, nullptr, nullptr);
-        else
-            srd::k_frag_gather_agg<false><<<f->final_grid, srd::GATHER_BLOCK, 0, ctx->stream>>>(fdev, (const srd::AggDev*)a->dev.p, pass, vt,
-                                                                                        f->sel[cur].as<srd::SelEntry>(), cnt + k, fail_list, fail_count);
-        SR_LAUNCH_CHECK(ctx);
+        SR_TRY(final_pass(f->sel[cur].as<srd::SelEntry>(), cnt + k, hash ? f->sel[cur ^ 1].as<srd::SelEntry>() : nullptr, cnt + 8));
         SR_CUDA(ctx, cudaEventRecord(f->ev[3], ctx->stream));
         f->timed_push = true;
         if (hash) {
@@ -558,15 +529,7 @@ static int32_t frag_push(sr_fragment* f, const sr_chunk_view* fact) {
                 cur ^= 1; // the fail list becomes the input, the old input buffer the new fail list
                 const int nfc = fc == 8 ? 9 : 8;
                 SR_CUDA(ctx, cudaMemsetAsync(cnt + nfc, 0, 8, ctx->stream));
-                if (f->expand)
-                    srd::k_frag_gather_agg_expand<<<f->final_grid, srd::GATHER_BLOCK, 0, ctx->stream>>>(fdev, (const srd::AggDev*)a->dev.p, pass, vt,
-                                                                                               f->sel[cur].as<srd::SelEntry>(), cnt + fc,
-                                                                                               f->sel[cur ^ 1].as<srd::SelEntry>(), cnt + nfc);
-                else
-                    srd::k_frag_gather_agg<false><<<f->final_grid, srd::GATHER_BLOCK, 0, ctx->stream>>>(fdev, (const srd::AggDev*)a->dev.p, pass, vt,
-                                                                                                f->sel[cur].as<srd::SelEntry>(), cnt + fc,
-                                                                                                f->sel[cur ^ 1].as<srd::SelEntry>(), cnt + nfc);
-                SR_LAUNCH_CHECK(ctx);
+                SR_TRY(final_pass(f->sel[cur].as<srd::SelEntry>(), cnt + fc, f->sel[cur ^ 1].as<srd::SelEntry>(), cnt + nfc));
                 fc = nfc;
             }
         }

@@ -36,15 +36,11 @@ struct PassDev {
     StreamTest tests[SR_MAX_STREAM_TESTS];
     int32_t num_stream_joins; // joins [0, num_stream_joins) are tested by the streaming pass
     int32_t final_first_join; // joins [final_first_join, S) are tested inline by the final pass
-    // fact columns the final pass reads: fetched for a row in one burst before anything depends on them
-    int8_t final_vals[8];              // value ids, -1 = unused
-    int8_t final_slot[SR_MAX_VALUES];  // value id -> index into final_vals, -1 = not prefetched
-    int8_t host_input; // the fact columns of this push live in pinned host memory (SR_MEM_HOST_PINNED)
     // the int32 key of one streamed join whose build row the final pass needs travels in the upper half of the
     // selection-vector entries, so the final pass does not gather it from the fact table again
     int8_t carry_join;     // index of that join among the streamed joins, -1 = none
     int8_t carry_value_id; // its key's value id
-    int8_t pad[1];
+    int8_t pad[2];
 };
 
 // selection-vector entry: row id (low 32 bits) + carried key (high 32 bits)
@@ -52,8 +48,6 @@ typedef unsigned long long SelEntry;
 __device__ __forceinline__ uint32_t sel_row(SelEntry e) { return (uint32_t)e; }
 __device__ __forceinline__ int32_t sel_carry(SelEntry e) { return (int32_t)(e >> 32); }
 __device__ __forceinline__ SelEntry sel_make(uint32_t row, int32_t carry) { return (SelEntry)row | ((SelEntry)(uint32_t)carry << 32); }
-
-#define SR_FINAL_PREFETCH 8
 
 // bitmap / hash test against the global copies only (gather passes do not stage bitmaps)
 __device__ __forceinline__ bool join_hit_global(const FragJoinDev& fj, int64_t key) {
@@ -118,11 +112,7 @@ __device__ __forceinline__ uint32_t join_test_batch(const FragJoinDev& fj, const
             for (int i = 0; i < N; i++) {
                 const uint32_t idx = (uint32_t)keys[i] - umin;
                 const bool p = ((alive >> i) & 1u) && idx <= span;
-#ifdef SR_EXPERIMENT_FAKE_SMEM
-                words[i] = p ? smem[(idx >> 5) & 4095u] : 0u; // timing experiment only: WRONG results
-#else
                 words[i] = ldg_u32_pred(fj.j.bitmap + (idx >> 5), p);
-#endif
             }
 #pragma unroll
             for (int i = 0; i < N; i++) {
@@ -232,6 +222,27 @@ __device__ __forceinline__ void warp_append_rows(uint32_t alive_all, int64_t row
     }
 }
 
+// prologue of both streaming kernels: the descriptors of the streamed joins [0, SJ) into s_joins, and their shared-memory
+// bitmaps into smem, each followed by the zero guard word that frag_plan reserves behind it (stream_test_reg kind 1)
+__device__ __forceinline__ void stream_stage_joins(const FragDev& fd, int SJ, FragJoinDev* s_joins, uint32_t* smem) {
+    for (int i = threadIdx.x; i < (int)(sizeof(FragJoinDev) / 4) * SJ; i += blockDim.x) ((uint32_t*)s_joins)[i] = ((const uint32_t*)fd.joins)[i];
+    for (int j = 0; j < SJ; j++) {
+        const FragJoinDev& fj = fd.joins[j];
+        if (fj.smem_off >= 0)
+            for (int w = threadIdx.x; w <= fj.bitmap_words; w += blockDim.x) smem[fj.smem_off + w] = w < fj.bitmap_words ? fj.j.bitmap[w] : 0u;
+    }
+}
+
+// Each CTA streams a CONTIGUOUS run of tiles [begin, end) (not a grid-stride walk): the rows a warp appends to one
+// selection-vector chunk then come from a narrow band of the table (~25 tiles) instead of being spread over the whole
+// batch, so the later gather passes touch neighbouring sectors / pages back to back.
+__device__ __forceinline__ void stream_tile_range(int64_t n, int64_t& begin, int64_t& end) {
+    const int64_t num_tiles = (n + STREAM_TILE - 1) / STREAM_TILE;
+    const int64_t tiles_per_cta = (num_tiles + gridDim.x - 1) / gridDim.x;
+    begin = (int64_t)blockIdx.x * tiles_per_cta;
+    end = begin + tiles_per_cta < num_tiles ? begin + tiles_per_cta : num_tiles;
+}
+
 // CARRY: the key of streamed join pd.carry_join rides in the upper half of the entries.  Only instantiated for
 // host-resident input: holding the tile's keys in registers through the append costs the streaming kernel ~25 %
 // when it runs at HBM speed (register spills; re-reading the key for the survivors instead was worse still, it puts
@@ -245,25 +256,15 @@ __global__ void __launch_bounds__(STREAM_BLOCK, 2) k_frag_stream(const FragDev* 
     __shared__ CPred s_preds[8];
     const FragDev& fd = *fdp;
     const int SJ = pd.num_stream_joins;
-    for (int i = threadIdx.x; i < (int)(sizeof(FragJoinDev) / 4) * SJ; i += blockDim.x) ((uint32_t*)s_joins)[i] = ((const uint32_t*)fd.joins)[i];
+    stream_stage_joins(fd, SJ, s_joins, smem);
     for (int i = threadIdx.x; i < (int)(sizeof(CPred) / 4) * fd.num_preds; i += blockDim.x) ((uint32_t*)s_preds)[i] = ((const uint32_t*)fd.preds)[i];
-    for (int j = 0; j < SJ; j++) {
-        const FragJoinDev& fj = fd.joins[j];
-        if (fj.smem_off >= 0)
-            for (int w = threadIdx.x; w < fj.bitmap_words; w += blockDim.x) smem[fj.smem_off + w] = fj.j.bitmap[w];
-    }
     __syncthreads();
 
     // (the common shapes -- range conjuncts and joins on plain int32 columns -- run in k_frag_stream_tests below;
     // this kernel is the general form: any predicate, generic filter expressions, nullable / wide key columns)
-    const int64_t num_tiles = (n + STREAM_TILE - 1) / STREAM_TILE;
     const int64_t full_tiles = n / STREAM_TILE;
-    // Each CTA streams a CONTIGUOUS run of tiles (not a grid-stride walk): the rows a warp appends to one
-    // selection-vector chunk then come from a narrow band of the table (~25 tiles) instead of being spread over
-    // the whole batch, so the later gather passes touch neighbouring sectors / pages back to back.
-    const int64_t tiles_per_cta = (num_tiles + gridDim.x - 1) / gridDim.x;
-    const int64_t tile_begin = (int64_t)blockIdx.x * tiles_per_cta;
-    const int64_t tile_end = tile_begin + tiles_per_cta < num_tiles ? tile_begin + tiles_per_cta : num_tiles;
+    int64_t tile_begin, tile_end;
+    stream_tile_range(n, tile_begin, tile_end);
     WarpSelWriter writer;
     writer.init(sel_out, counter);
 
@@ -444,13 +445,8 @@ __global__ void __launch_bounds__(STREAM_BLOCK, 2) k_frag_stream_tests(const Fra
     const int SJ = pd.num_stream_joins;
     const int NT = pd.num_tests;
     const int NV = pd.num_vec;
-    for (int i = threadIdx.x; i < (int)(sizeof(FragJoinDev) / 4) * SJ; i += blockDim.x) ((uint32_t*)s_joins)[i] = ((const uint32_t*)fd.joins)[i];
+    stream_stage_joins(fd, SJ, s_joins, smem);
     for (int i = threadIdx.x; i < (int)(sizeof(StreamTest) / 4) * NT; i += blockDim.x) ((uint32_t*)s_tests)[i] = ((const uint32_t*)pd.tests)[i];
-    for (int j = 0; j < SJ; j++) {
-        const FragJoinDev& fj = fd.joins[j];
-        if (fj.smem_off >= 0) // + the zero guard word behind the copy (frag_plan reserves it)
-            for (int w = threadIdx.x; w <= fj.bitmap_words; w += blockDim.x) smem[fj.smem_off + w] = w < fj.bitmap_words ? fj.j.bitmap[w] : 0u;
-    }
     __syncthreads();
     const TestReg t0 = make_test_reg(s_tests[0], s_joins, smem);
     const TestReg t1 = make_test_reg(s_tests[NV > 1 ? 1 : 0], s_joins, smem);
@@ -458,11 +454,9 @@ __global__ void __launch_bounds__(STREAM_BLOCK, 2) k_frag_stream_tests(const Fra
     const bool carry1 = CARRY && NV > 1 && s_tests[1].kind == 1 && s_tests[1].join == pd.carry_join;
     const int32_t* col0 = (const int32_t*)vt.v[pd.tests[0].value_id].data;
     const int32_t* col1 = NV > 1 ? (const int32_t*)vt.v[pd.tests[1].value_id].data : nullptr;
-    const int64_t num_tiles = (n + STREAM_TILE - 1) / STREAM_TILE;
     const int64_t full_tiles = n / STREAM_TILE;
-    const int64_t tiles_per_cta = (num_tiles + gridDim.x - 1) / gridDim.x;
-    const int64_t tile_begin = (int64_t)blockIdx.x * tiles_per_cta;
-    const int64_t tile_end = tile_begin + tiles_per_cta < num_tiles ? tile_begin + tiles_per_cta : num_tiles;
+    int64_t tile_begin, tile_end;
+    stream_tile_range(n, tile_begin, tile_end);
     const int64_t prefetch_end = tile_end < full_tiles ? tile_end : full_tiles;
     int4 pk[2][STREAM_GROUPS];
 #pragma unroll
@@ -507,158 +501,6 @@ __global__ void __launch_bounds__(STREAM_BLOCK, 2) k_frag_stream_tests(const Fra
             if (NV > 1) {
                 a8 = stream_test_reg<8>(t1, s_tests[1], s_joins, smem, k1, a8);
                 if (carry1) {
-#pragma unroll
-                    for (int i = 0; i < 8; i++) carry[i] = k1[i];
-                }
-            }
-            first_pred = NV;
-        } else { // the ragged last tile: every test through predicated loads
-            a8 = 0;
-#pragma unroll
-            for (int i = 0; i < 8; i++)
-                if (row0[i >> 2] + (i & 3) < n) a8 |= 1u << i;
-        }
-#pragma unroll 1
-        for (int t = first_pred; t < NT; t++) {
-            const StreamTest& st = s_tests[t];
-            const int32_t* col = (const int32_t*)vt.v[st.value_id].data;
-            int32_t kk[8];
-#pragma unroll
-            for (int i = 0; i < 8; i++) kk[i] = ldg_stream_s32_pred(col + row0[i >> 2] + (i & 3), (a8 >> i) & 1u);
-            a8 = stream_test<8>(st, s_joins, smem, kk, a8);
-            if (CARRY && st.kind == 1 && st.join == pd.carry_join) {
-#pragma unroll
-                for (int i = 0; i < 8; i++) carry[i] = kk[i];
-            }
-        }
-        warp_append_rows<CARRY>(a8, row0[0], row0[1], carry, writer);
-    }
-    writer.finish();
-}
-
-// ---- the same pass with the vector columns staged by the TMA engine (north_star: "TMA-staged into shared memory") ----
-// The tile's two vector columns (STREAM_TILE x 4 bytes each) are fetched with cp.async.bulk (1-D bulk copy, SASS UBLKCP)
-// into a two-stage ring in shared memory, completion signalled through an mbarrier (complete_tx::bytes); the threads read
-// their eight keys per column with 128-bit shared loads and release the stage through a second mbarrier, on which thread 0
-// waits before it issues the copy of tile + 2.  The register prefetch of k_frag_stream_tests and its LDG.128 / L1TEX tag
-// traffic are gone; the price is 64 KB more shared memory per CTA and two shared loads per column.
-// Opt-in (SR_FRAG_STREAM_TMA=1): measured against the LDG form in profiles/r2_notes.md.
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"((uint32_t)__cvta_generic_to_shared(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"((uint32_t)__cvta_generic_to_shared(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"((uint32_t)__cvta_generic_to_shared(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-    asm volatile(
-            "{ .reg .pred p;\n"
-            "WAIT_%=:\n"
-            "  mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-            "  @p bra DONE_%=;\n"
-            "  bra WAIT_%=;\n"
-            "DONE_%=: }" ::"r"((uint32_t)__cvta_generic_to_shared(bar)),
-            "r"(parity)
-            : "memory");
-}
-__device__ __forceinline__ void tma_load_1d(void* smem_dst, const void* gmem_src, uint32_t bytes, uint64_t* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"((uint32_t)__cvta_generic_to_shared(smem_dst)),
-                 "l"(gmem_src), "r"(bytes), "r"((uint32_t)__cvta_generic_to_shared(bar))
-                 : "memory");
-}
-
-constexpr int STREAM_TMA_STAGES = 2;
-constexpr size_t STREAM_TMA_SMEM = (size_t)STREAM_TMA_STAGES * 2 * STREAM_TILE * sizeof(int32_t);
-
-// smem: [bitmaps: bitmap_bytes][stage 0: col0 tile, col1 tile][stage 1: ...]; bitmap_bytes is a multiple of 16
-template <bool CARRY>
-__global__ void __launch_bounds__(STREAM_BLOCK, 2) k_frag_stream_tests_tma(const FragDev* __restrict__ fdp, PassDev pd, const __grid_constant__ VTab vt, int64_t n,
-                                                                           uint32_t bitmap_bytes, SelEntry* __restrict__ sel_out, unsigned long long* __restrict__ counter) {
-    extern __shared__ __align__(128) uint32_t smem_tma[];
-    uint32_t* const smem = smem_tma;
-    __shared__ FragJoinDev s_joins[STREAM_MAX_JOINS];
-    __shared__ StreamTest s_tests[SR_MAX_STREAM_TESTS];
-    __shared__ __align__(8) uint64_t s_full[STREAM_TMA_STAGES], s_empty[STREAM_TMA_STAGES];
-    const FragDev& fd = *fdp;
-    const int SJ = pd.num_stream_joins;
-    const int NT = pd.num_tests;
-    const int NV = pd.num_vec;
-    for (int i = threadIdx.x; i < (int)(sizeof(FragJoinDev) / 4) * SJ; i += blockDim.x) ((uint32_t*)s_joins)[i] = ((const uint32_t*)fd.joins)[i];
-    for (int i = threadIdx.x; i < (int)(sizeof(StreamTest) / 4) * NT; i += blockDim.x) ((uint32_t*)s_tests)[i] = ((const uint32_t*)pd.tests)[i];
-    for (int j = 0; j < SJ; j++) {
-        const FragJoinDev& fj = fd.joins[j];
-        if (fj.smem_off >= 0)
-            for (int w = threadIdx.x; w < fj.bitmap_words; w += blockDim.x) smem[fj.smem_off + w] = fj.j.bitmap[w];
-    }
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < STREAM_TMA_STAGES; s++) {
-            mbar_init(&s_full[s], 1);
-            mbar_init(&s_empty[s], STREAM_BLOCK);
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    int32_t* const ring = (int32_t*)((uint8_t*)smem + bitmap_bytes);
-    const int32_t* col0 = (const int32_t*)vt.v[pd.tests[0].value_id].data;
-    const int32_t* col1 = NV > 1 ? (const int32_t*)vt.v[pd.tests[1].value_id].data : nullptr;
-    const int64_t num_tiles = (n + STREAM_TILE - 1) / STREAM_TILE;
-    const int64_t full_tiles = n / STREAM_TILE;
-    const int64_t tiles_per_cta = (num_tiles + gridDim.x - 1) / gridDim.x;
-    const int64_t tile_begin = (int64_t)blockIdx.x * tiles_per_cta;
-    const int64_t tile_end = tile_begin + tiles_per_cta < num_tiles ? tile_begin + tiles_per_cta : num_tiles;
-    const int64_t tma_end = tile_end < full_tiles ? tile_end : full_tiles; // full tiles only; the ragged tail uses predicated loads
-    const uint32_t col_bytes = STREAM_TILE * sizeof(int32_t);
-    auto issue = [&](int64_t tile) { // thread 0 only
-        const int s = (int)((tile - tile_begin) % STREAM_TMA_STAGES);
-        mbar_expect_tx(&s_full[s], col1 ? 2 * col_bytes : col_bytes);
-        tma_load_1d(ring + (size_t)s * 2 * STREAM_TILE, col0 + tile * STREAM_TILE, col_bytes, &s_full[s]);
-        if (col1) tma_load_1d(ring + (size_t)s * 2 * STREAM_TILE + STREAM_TILE, col1 + tile * STREAM_TILE, col_bytes, &s_full[s]);
-    };
-    if (threadIdx.x == 0)
-        for (int64_t t = tile_begin; t < tma_end && t < tile_begin + STREAM_TMA_STAGES; t++) issue(t);
-    WarpSelWriter writer;
-    writer.init(sel_out, counter);
-    for (int64_t tile = tile_begin; tile < tile_end; tile++) {
-        int64_t row0[STREAM_GROUPS];
-#pragma unroll
-        for (int g = 0; g < STREAM_GROUPS; g++)
-            row0[g] = tile * STREAM_TILE + (int64_t)g * (STREAM_BLOCK * STREAM_ROWS) + (int64_t)threadIdx.x * STREAM_ROWS;
-        int32_t carry[8];
-        if (CARRY) {
-#pragma unroll
-            for (int i = 0; i < 8; i++) carry[i] = 0;
-        }
-        uint32_t a8 = 0xFFu;
-        int first_pred = 0;
-        if (tile < tma_end) {
-            const int64_t li = tile - tile_begin;
-            const int s = (int)(li % STREAM_TMA_STAGES);
-            const uint32_t parity = (uint32_t)((li / STREAM_TMA_STAGES) & 1);
-            mbar_wait(&s_full[s], parity);
-            const int32_t* st0 = ring + (size_t)s * 2 * STREAM_TILE;
-            const int4 a0 = *(const int4*)(st0 + threadIdx.x * STREAM_ROWS), a1 = *(const int4*)(st0 + STREAM_BLOCK * STREAM_ROWS + threadIdx.x * STREAM_ROWS);
-            int4 b0 = make_int4(0, 0, 0, 0), b1 = make_int4(0, 0, 0, 0);
-            if (col1) {
-                b0 = *(const int4*)(st0 + STREAM_TILE + threadIdx.x * STREAM_ROWS);
-                b1 = *(const int4*)(st0 + STREAM_TILE + STREAM_BLOCK * STREAM_ROWS + threadIdx.x * STREAM_ROWS);
-            }
-            mbar_arrive(&s_empty[s]); // this thread has its keys in registers
-            if (threadIdx.x == 0 && tile + STREAM_TMA_STAGES < tma_end) {
-                mbar_wait(&s_empty[s], parity); // every thread has read the stage: refill it with tile + 2
-                issue(tile + STREAM_TMA_STAGES);
-            }
-            const int32_t k0[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
-            const int32_t k1[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
-            a8 = stream_test<8>(s_tests[0], s_joins, smem, k0, 0xFFu);
-            if (CARRY && s_tests[0].kind == 1 && s_tests[0].join == pd.carry_join) {
-#pragma unroll
-                for (int i = 0; i < 8; i++) carry[i] = k0[i];
-            }
-            if (NV > 1) {
-                a8 = stream_test<8>(s_tests[1], s_joins, smem, k1, a8);
-                if (CARRY && s_tests[1].kind == 1 && s_tests[1].join == pd.carry_join) {
 #pragma unroll
                     for (int i = 0; i < 8; i++) carry[i] = k1[i];
                 }
@@ -745,6 +587,29 @@ __global__ void __launch_bounds__(GATHER_BLOCK) k_frag_gather_join(const FragDev
     writer.finish();
 }
 
+// the joins of one row in the final pass: joins [final_first_join, S) are tested, and every join whose build row is read
+// downstream (or that has no bitmap) leaves its chain head in ld.bidx -- the other entries keep the 0 they start with.
+// false: the row fails a tested join
+__device__ __forceinline__ bool final_join_walk(const FragJoinDev* s_joins, int S, int final_first_join, FragLoader& ld) {
+#pragma unroll 1
+    for (int j = 0; j < S; j++) {
+        const FragJoinDev& fj = s_joins[j];
+        const bool test = j >= final_first_join;
+        if (!test && !fj.need_head) continue;
+        int64_t key;
+        const bool nul = ld.load(fj.key_value_id, key);
+        if (test && nul) return false;
+        if (fj.need_head || !fj.use_bitmap) {
+            const uint32_t head = join_lookup(fj.j, key);
+            ld.bidx[j] = head;
+            if (test && head == 0) return false;
+        } else if (test && !join_hit_global(fj, key)) {
+            return false;
+        }
+    }
+    return true;
+}
+
 // final pass: remaining joins inline, payload lookups, aggregate update.  SINGLE: no GROUP BY (its register state
 // would only cost the grouped instantiations spills).
 template <bool SMEM_AGG, bool SINGLE = false>
@@ -790,27 +655,7 @@ __global__ void __launch_bounds__(GATHER_BLOCK, SR_GATHER_AGG_MIN_BLOCKS) k_frag
         // (a variant that fetched every fact value of the row in one burst before the dependent lookups was
         // measured slower on B200 -- more issue slots and registers than latency hidden, see profiles/)
         FragLoader ld{vt, (int64_t)row, {0, 0, 0, 0, 0, 0}, pd.carry_join >= 0 ? (int32_t)pd.carry_value_id : -1, sel_carry(entry)};
-        bool ok = true;
-#pragma unroll 1
-        for (int j = 0; j < S && ok; j++) {
-            const FragJoinDev& fj = s_joins[j];
-            const bool test = j >= pd.final_first_join;
-            if (!test && !fj.need_head) continue;
-            int64_t key;
-            const bool nul = ld.load(fj.key_value_id, key);
-            if (test && nul) {
-                ok = false;
-                break;
-            }
-            if (fj.need_head || !fj.use_bitmap) {
-                const uint32_t head = join_lookup(fj.j, key);
-                ld.bidx[j] = head;
-                if (test && head == 0) ok = false;
-            } else if (test) {
-                if (!join_hit_global(fj, key)) ok = false;
-            }
-        }
-        if (!ok) continue;
+        if (!final_join_walk(s_joins, S, pd.final_first_join, ld)) continue;
         if (single) { // no GROUP BY: the state lives in the thread, not behind an atomic
             single_acc_row(ad, sacc, ld);
         } else if (hash_table) {
@@ -873,29 +718,10 @@ __global__ void __launch_bounds__(GATHER_BLOCK) k_frag_gather_agg_expand(const F
         const uint32_t row = sel_row(entry);
         if (row == SEL_INVALID) continue;
         FragLoader ld{vt, (int64_t)row, {0, 0, 0, 0, 0, 0}, pd.carry_join >= 0 ? (int32_t)pd.carry_value_id : -1, sel_carry(entry)};
+        if (!final_join_walk(s_joins, S, pd.final_first_join, ld)) continue;
         uint32_t head[SR_MAX_FRAG_JOINS];
-        bool ok = true;
 #pragma unroll 1
-        for (int j = 0; j < S && ok; j++) {
-            const FragJoinDev& fj = s_joins[j];
-            head[j] = 0;
-            const bool test = j >= pd.final_first_join;
-            if (!test && !fj.need_head) continue;
-            int64_t key;
-            const bool nul = ld.load(fj.key_value_id, key);
-            if (test && nul) {
-                ok = false;
-                break;
-            }
-            if (fj.need_head || !fj.use_bitmap) {
-                head[j] = join_lookup(fj.j, key);
-                ld.bidx[j] = head[j];
-                if (test && head[j] == 0) ok = false;
-            } else if (test) {
-                if (!join_hit_global(fj, key)) ok = false;
-            }
-        }
-        if (!ok) continue;
+        for (int j = 0; j < S; j++) head[j] = ld.bidx[j];
         bool refused = false;
 #pragma unroll 1
         for (int phase = hash_table ? 0 : 1; phase < 2 && !refused; phase++) {

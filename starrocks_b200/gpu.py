@@ -42,7 +42,7 @@ def build(verbose=False):
     (the ranks of a torchrun job): one process compiles under a file lock into a temporary name and renames it into place."""
     import fcntl
     src = os.path.join(_HERE, "csrc", "sr_gpu.cu")
-    extra = os.environ.get("SR_NVCC_EXTRA", "").split()   # e.g. -DSR_EXPERIMENT_... for timing experiments
+    extra = os.environ.get("SR_NVCC_EXTRA", "").split()   # e.g. -DSR_GATHER_AGG_MIN_BLOCKS=4 for timing experiments
     want = _source_hash()
     with open(LIB_PATH + ".lock", "w") as lock:
         fcntl.flock(lock, fcntl.LOCK_EX)
